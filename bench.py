@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mpix/s of dense DIS flow on synthetic 1024x436 pairs (op-point 2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (all pyramid levels: patch inverse search,
 densification, variational refinement == the reference's "O.Flow Run-Time"
@@ -308,6 +308,17 @@ def measure_sharded(args, prm, rank, world, local, stream, barrier, maxrank):
     return out
 
 
+def dump_flows(out_dir, ctx, B, li, prm, limit=64 << 20):
+    """What a caller of the resident path receives from `ctx`'s last run: the flow of level sc_l of every pair, as
+    DIR/flow.npy; the first pairs only when all of them would exceed `limit` bytes."""
+    n = min(B, limit // (li["h"] * li["w"] * prm.nop * 4))
+    flow = np.empty((n, li["h"], li["w"], prm.nop), np.float32)
+    ctx.get_flow_batch(0, n, flow)
+    ctx.sync()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "flow.npy"), flow)
+
+
 def measure_big_configs():
     """BASELINE configs[2] and configs[4] on this GPU (tools/big_configs.py): step time, per kernel
     class and per level; the SOR of configs[4]'s level 1 at 8 pairs is the launch SURVEY 8(d) names."""
@@ -342,7 +353,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the sharded and big_configs legs")
     ap.add_argument("--opt", action="append", default=[], metavar="NAME=VALUE",
                     help="ofdis_set_option on every context (launch-geometry experiments; results are bit-identical)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the flows the last one computed as DIR/flow.npy (float32, "
+                         "[pair][h][w][nop] at level sc_l; rank 0's pairs, the first ones only beyond 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path")
     args.warmup = max(args.warmup, 3)
     if args.lanes <= 0:
         divs = [d for d in range(6, 13) if args.steps % d == 0]
@@ -458,6 +474,8 @@ def main():
     t0 = time.time()
     ms_res = maxrank(pipelined(resident_step, args.steps))
     launches = (sum(l[0].launch_count for l in lanes) - l0) // args.steps
+    if args.dump_outputs and rank == 0:
+        dump_flows(args.dump_outputs, lanes[(args.steps - 1) % NL][0], B, li, prm)
     barrier()
     # The K timed steps above last a few milliseconds.  The same loop over >= 0.5 s: clocks and thermals under a
     # sustained load (the clock sampler runs through both), reported beside `value`, never instead of it.

@@ -6,7 +6,9 @@ container that has /root/reference:
 
 Each fixture holds the uint8 input pair, the parameters (20 CLI numbers + noc +
 nop) and the reference flow at level sc_l, plus the patch-stage outputs of the
-finest level (p, conv, cnt) for a fixed seeded coarser flow.
+finest level (p, conv, cnt) for a fixed seeded coarser flow.  reference/runs.npz
+keeps, for the larger cases tests/test_oracle.py compares with the reference, the
+shape, SHA-256 and a seeded sample of each reference output.
 """
 import os
 import sys
@@ -34,9 +36,26 @@ CASES = {
 }
 
 
+def reference_runs(out_dir):
+    """reference/runs.npz: digests and samples of what the reference build computes for the cases
+    tests/test_oracle.py compares the port with (test_oracle.REFERENCE_CASES)."""
+    sys.path.insert(0, os.path.dirname(out_dir))
+    import test_oracle
+
+    out = {}
+    for name in test_oracle.REFERENCE_CASES:
+        case = test_oracle.reference_case(name)
+        out.update(test_oracle.summarize(case, test_oracle.reference_outputs(case)))
+        print(name)
+    os.makedirs(os.path.join(out_dir, "reference"), exist_ok=True)
+    np.savez_compressed(os.path.join(out_dir, "reference", "runs.npz"), **out)
+
+
 def main():
     out_dir = os.path.dirname(os.path.abspath(__file__))
-    only = sys.argv[1:]  # optional: generate just these fixtures
+    only = sys.argv[1:]  # optional: generate just these fixtures ("reference" = reference/runs.npz)
+    if not only or "reference" in only:
+        reference_runs(out_dir)
     for name, (h, w, ch, cli, nop, amp, stereo) in CASES.items():
         if only and name not in only:
             continue

@@ -132,7 +132,7 @@ def test_sharded_engine_on_nccl_with_the_real_engine(io, nfr):
     """BASELINE configs[3] in miniature on two GPUs: rank 0 scatters the pairs over NCCL, both ranks run the
     CUDA engine, rank 0 gathers -- bitwise equal to the single-GPU result (equal and unequal blocks)."""
     if not torch.cuda.is_available() or torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29700 + (os.getpid() % 2000) + nfr

@@ -2,8 +2,8 @@
 one GPU: step time and, per kernel class, the achieved algorithmic GB/s (SURVEY 8d formulas) -- the
 levels of these configs are the ones that stream from HBM.  Also the SOR time per pyramid level.
 python tools/big_configs.py [B ...] [--opt name=value ...] [--cfg substring]"""
-import sys, time, json
-sys.path.insert(0, '/root/repo')
+import os, sys, time, json
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 from of_dis_b200 import api, params, preprocess, synth

@@ -1,6 +1,6 @@
 """Which part of the e2e step breaks the overlap between lanes?  A/B variants on one box."""
-import sys, time
-sys.path.insert(0, '/root/repo')
+import os, sys, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from of_dis_b200 import api, params, preprocess, synth
 prm = params.operating_point(2, 1024)

@@ -1,6 +1,7 @@
 """1920x1080 gray at operating point 2 (levels 6..4, finest 240x135... see level_info): lane step time."""
+import os
 import sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from of_dis_b200 import api, params, preprocess, synth
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 16

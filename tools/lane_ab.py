@@ -2,9 +2,10 @@
 configs[2] (1920x1080 RGB): ofdis_set_option("sor_lane", 0 | 1); per pyramid level the SOR and assemble time of
 one eager pass, and the graph-replayed step time.  python tools/lane_ab.py [B ...]  -> one JSON line per (config, B, lane)."""
 import json
+import os
 import sys
 
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 from of_dis_b200 import api, params, synth

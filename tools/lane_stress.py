@@ -2,9 +2,10 @@
 inputs, every flow compared bit for bit with the first one (a memory-ordering bug would be a rare event, not a
 deterministic one).  python tools/lane_stress.py [replays]"""
 import json
+import os
 import sys
 
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from of_dis_b200 import api, params, preprocess, synth
 

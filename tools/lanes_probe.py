@@ -1,6 +1,6 @@
 """Resident throughput of NL lanes (graph replay), for A/B experiments driven by env knobs."""
-import sys, time
-sys.path.insert(0, '/root/repo')
+import os, sys, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from of_dis_b200 import api, params, preprocess, synth
 import dataclasses, os

@@ -1,6 +1,6 @@
 """H2D/D2H rate of a pinned 8 MB buffer allocated on each NUMA node of the host (A/B on one box)."""
 import os, sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from of_dis_b200 import numa
 torch.cuda.set_device(0)

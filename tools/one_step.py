@@ -1,8 +1,9 @@
 """One eager step (48 launches at operating point 2) of a B-pair batch, for ncu launch lists:
    ncu --metrics gpu__time_duration.sum,smsp__inst_executed.sum --clock-control none --csv \
        --log-file gpurun_out/x.csv python tools/one_step.py [B] [steps]"""
+import os
 import sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from of_dis_b200 import api, params, preprocess, synth
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 64

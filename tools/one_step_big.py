@@ -1,9 +1,10 @@
 """One eager step of BASELINE configs[2] (cfg3) or configs[4] (cfg5) on B pairs, for ncu captures of the
 P = 12 patch kernel and the cluster SOR:
    ncu --set full -k regex:sor_wave -c 3 ... python tools/one_step_big.py cfg5 1"""
+import os
 import sys
-sys.path.insert(0, '/root/repo')
-sys.path.insert(0, '/root/repo/tools')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import numpy as np
 from of_dis_b200 import api, synth
 import big_configs

@@ -2,10 +2,11 @@
 of 1 / 8 / 64 pairs on one stream, flows compared bit for bit; a second pass runs 20 replays each and compares all.
 python tools/pdl_ab.py [B ...]"""
 import json
+import os
 import sys
 import time
 
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from of_dis_b200 import api, params, synth
 
