@@ -210,9 +210,7 @@ int ofdis_set_direction(ofdis_ctx* ctx, int dir);
  *                     (a level needs W/4 + h/rows super-steps; sor_wave_kernel.cuh)
  *   "sor_single_max"  32 | 64 | 128 (default): refinement levels of up to this many SOR lanes (= rows / rows per
  *                     thread) run their SOR in one CTA, taller ones in a thread-block cluster of row bands
- *   "sor_max_cluster" 8 (portable) | 16 (default where the device grants it)
- *   "patch_window_tma" 0 (default) | 1: the P = 12 patch kernel fills its shared-memory I1 window with a TMA
- *                     tensor tile copy instead of LDG+STS on levels whose row pitch is a multiple of 16 bytes */
+ *   "sor_max_cluster" 8 (portable) | 16 (default where the device grants it) */
 int ofdis_set_option(ofdis_ctx* ctx, const char* name, int value);
 /* CUDA-graph replay of ofdis_run (captured on first use per nframes). */
 int ofdis_set_graph_mode(ofdis_ctx* ctx, int enabled);

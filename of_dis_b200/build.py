@@ -43,9 +43,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not needs_build():
         return LIB
     os.makedirs(LIBDIR, exist_ok=True)
-    extra = ["-DOFDIS_SOR_TIMING"] if os.environ.get("OFDIS_SOR_TIMING") else []
-    extra += ["-D" + d for d in os.environ.get("OFDIS_EXP_DEFINES", "").split()]  # experiment builds of tools/ only
-    cmd = [_nvcc()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + \
+    cmd = [_nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + \
           [os.path.join(CSRC, s) for s in SOURCES] + ["-ldl", "-o", LIB]  # -ldl: NVTX v3 loads its injection library lazily
     res = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or res.returncode:

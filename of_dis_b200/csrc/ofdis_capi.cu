@@ -244,7 +244,6 @@ int ofdis_create(ofdis_ctx** out, int device, void* stream, const ofdis_params* 
   ctx->pp.dp_thresh_sq = prm->dp_thresh * prm->dp_thresh;  // oflow.cpp:88
   ctx->pp.dr_thresh = prm->dr_thresh;
   ctx->pp.res_thresh = prm->res_thresh;
-  ctx->pp.window_tma = 0;
 
   // geometry + packed image layout: per frame, level sc_f down to sc_l, I0 I0x I0y I1
   ctx->lev.resize(ctx->nlev);
@@ -739,9 +738,6 @@ int ofdis_set_option(ofdis_ctx* ctx, const char* name, int value) {
       ctx->planes.fdu = ctx->d_fast + plane * 8 * ctx->cap;
     }
     ctx->planes.fast = value;
-  } else if (!strcmp(name, "patch_window_tma")) {
-    if (value != 0 && value != 1) return fail(ctx, OFDIS_ERR_ARG, "patch_window_tma: 0 or 1");
-    ctx->pp.window_tma = value;
   } else if (!strcmp(name, "sor_rows_per_thread")) {
     if (value != 1 && value != 2 && value != 4) return fail(ctx, OFDIS_ERR_ARG, "sor_rows_per_thread: 1, 2 or 4");
     VarRefPlanes probe{};

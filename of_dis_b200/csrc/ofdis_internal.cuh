@@ -43,7 +43,6 @@ __host__ __device__ __forceinline__ int camlr_of(const LevelGeom& g, int frame) 
 struct PatchParams {
   int max_iter, min_iter, costfct, patnorm;
   float dp_thresh_sq, dr_thresh, res_thresh;
-  int window_tma;  // P = 12 kernel: fill the I1 window with a TMA tensor tile copy where the level's pitch allows it
 };
 
 // Refinement workspace for one level (all frames), planar planes of pitch*h floats.

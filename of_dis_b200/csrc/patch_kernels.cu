@@ -14,11 +14,6 @@
 // [slot][thread] columns (conflict free, private to the thread), staged once.
 // The bilinear taps of I1 are plain LDGs: the (P+1)x(P+1) window of a patch
 // moves by a fraction of a pixel per iteration and stays L1-resident.
-#include <cstdint>
-#include <cstring>
-
-#include <cuda.h>  // CUtensorMap (types only; the encoder is fetched through cudaGetDriverEntryPoint)
-
 #include "ofdis_internal.cuh"
 
 namespace ofdis {
@@ -529,59 +524,34 @@ __global__ void __launch_bounds__(256) patch_p8c1_kernel(LevelGeom g, PatchParam
 //   * element offsets are walked incrementally (no offset table).
 // Arithmetic (operand order, reduction tree, stop tests) is that of patch_optimize_kernel.
 //
-// TMA = true is the north-star's variant of the window fill: one lane of the patch issues a tensor
-// tile copy (cp.async.bulk.tensor.3d -> UTMALDG; box = window, coordinates (x*C, y, frame) in a
-// tensor map over the padded I1 frames, out-of-image cells zero-filled by the TMA unit) and the
-// patch's 8 lanes wait on an mbarrier, instead of 8 lanes x ~37 LDG+STS.  Tensor-map rules found the
-// hard way (tools/probe/tma_probe.cu): the row pitch of the padded image must be a multiple of 16
-// bytes (most level widths w+2P are not: only some levels qualify), the box's inner extent too, the
-// window must be 128-byte aligned in shared memory, and -- undocumented, "illegal instruction"
-// otherwise -- the box's START along the inner dimension must be 16-byte aligned as well, i.e. the
-// window's left edge sits on a multiple of 4 pixels and the window grows from 17 to 20 pixels.
-// A/B in DESIGN.md section 5 (ofdis_set_option "patch_window_tma").
+// The window is filled with LDG: a TMA tensor-tile fill was measured and loses (DESIGN.md section 5.2).
 template <int V> struct CostTag { static constexpr int value = V; };
-template <int C> struct PwCfg {
-  static constexpr int P = 12, M = 2, W = P + 1 + 2 * M, WC = W * C, PC = P * C, N = P * P * C, NK = N / 8;
-  static constexpr int WT = W + 3;              // TMA: window width (pixels): left edge on a multiple of 4 pixels
-  static constexpr int WCB = WT * C;            // TMA: window row pitch (floats) = inner box extent, a multiple of 4
-};
-template <int NOP, int C, bool TMA> struct PwWin {
-  static constexpr int WH = (NOP == 2) ? PwCfg<C>::W : PwCfg<C>::P + 1;          // window rows
-  static constexpr int PITCH = TMA ? PwCfg<C>::WCB : PwCfg<C>::WC;               // floats per window row
-  static constexpr int WIN = TMA ? (WH * PITCH * 4 + 127) / 128 * 32 : WH * PITCH;  // floats per window (TMA: 128-byte aligned)
+template <int NOP, int C> struct PwCfg {
+  static constexpr int P = 12, M = 2, W = P + 1 + 2 * M, PC = P * C, N = P * P * C, NK = N / 8;
+  static constexpr int WH = (NOP == 2) ? W : P + 1;  // window rows
+  static constexpr int WC = W * C;                    // floats per window row
+  static constexpr int WIN = WH * WC;                 // floats per window
 };
 
-template <int NOP, int C, bool TMA>
+template <int NOP, int C>
 __global__ void __launch_bounds__(256, C == 1 ? 2 : 1) patch_p12_kernel(LevelGeom g, PatchParams pp, int f0,
-                                                                        int init_from_coarser,
-                                                                        const __grid_constant__ CUtensorMap tmap) {
+                                                                        int init_from_coarser) {
   pdl_wait();  // programmatic dependent launch: nothing of the previous kernel is touched before this
-  using Cfg = PwCfg<C>;
-  constexpr int P = Cfg::P, M = Cfg::M, W = Cfg::W, PC = Cfg::PC, NK = Cfg::NK;
-  constexpr int WH = PwWin<NOP, C, TMA>::WH;    // window rows
-  constexpr int WC = PwWin<NOP, C, TMA>::PITCH;  // floats per window row
-  constexpr int WIN = PwWin<NOP, C, TMA>::WIN;  // floats per window
+  using Cfg = PwCfg<NOP, C>;
+  constexpr int P = Cfg::P, M = Cfg::M, W = Cfg::W, PC = Cfg::PC, N = Cfg::N, NK = Cfg::NK;
+  constexpr int WH = Cfg::WH, WC = Cfg::WC, WIN = Cfg::WIN;
+  constexpr int SY = WH - P - 1;  // rows of slack (stereo: none, the row never moves)
   constexpr bool G_REG = (C == 1);            // template gradients in registers
-  extern __shared__ __align__(128) float smem[];
+  extern __shared__ float smem[];
   const int tid = threadIdx.x, nthr = blockDim.x;
   const int l8 = tid & 7;
   const int frame = f0 + blockIdx.y;
   const int ip = blockIdx.x * (nthr >> 3) + (tid >> 3);
   const bool valid = ip < g.np;
-  const float fn = (float)Cfg::N;
+  const float fn = (float)N;
   float* const win = smem + (tid >> 3) * WIN;                  // this patch's window
   float* const sGx = smem + (nthr >> 3) * WIN + tid;           // RGB: gradient columns [k][thread]
   float* const sGy = sGx + NK * nthr;
-  // TMA: one mbarrier per patch behind the windows (and the gradient columns)
-  const unsigned mbar = (unsigned)__cvta_generic_to_shared(smem + (nthr >> 3) * WIN + (G_REG ? 0 : 2 * NK * nthr)) + 8u * (tid >> 3);
-  unsigned wphase = 0;
-  if (TMA) {
-    if (l8 == 0) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(mbar), "r"(1u) : "memory");
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-  }
   const int rowC = g.tmp_w * C;
 
   const float* i0 = g.img[0] + (size_t)frame * g.img_fs[0];
@@ -704,37 +674,15 @@ __global__ void __launch_bounds__(256, C == 1 ? 2 : 1) patch_p12_kernel(LevelGeo
         const int tx = pcx + g.pad - P / 2 - 1, ty = pcy + g.pad - P / 2 - 1;
         ux = tx - wx0;
         uy = ty - wy0;
-        restage = (ux < 0) | (ux > 2 * M + (TMA ? 3 : 0)) | (uy < 0) | (uy > ((NOP == 2) ? 2 * M : 0));
+        restage = (ux < 0) | (ux > W - P - 1) | (uy < 0) | (uy > SY);
         if (restage) {
-          wx0 = TMA ? ((tx - M) >> 2) << 2 : tx - M;  // TMA: the box must start on a 16-byte boundary
+          wx0 = tx - M;
           wy0 = (NOP == 2) ? ty - M : ty;
           ux = tx - wx0;
           uy = (NOP == 2) ? M : 0;
         }
       }
-      if (TMA) {
-        if (__any_sync(FULL, restage)) {
-          __syncwarp();  // every lane has finished reading the previous window
-          if (restage) {
-            if (l8 == 0) {
-              const unsigned dst = (unsigned)__cvta_generic_to_shared(win);
-              // the lanes' generic-proxy reads of the old window come before the async-proxy write
-              asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-              asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"((unsigned)(WH * WC * 4)) : "memory");
-              asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                           ::"r"(dst), "l"(&tmap), "r"(mbar), "r"(wx0 * C), "r"(wy0), "r"(frame)
-                           : "memory");
-            }
-            asm volatile(
-                "{\n\t.reg .pred p;\n\tPW_%=:\n\t"
-                "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                "@p bra PD_%=;\n\tbra PW_%=;\n\tPD_%=:\n\t}" ::"r"(mbar), "r"(wphase)
-                : "memory");
-            wphase ^= 1u;
-          }
-          __syncwarp();
-        }
-      } else if (__any_sync(FULL, restage)) {
+      if (__any_sync(FULL, restage)) {
         __syncwarp();  // every lane has finished reading the previous window
         if (restage) {
           const int xlo = wx0 * C, xmax = g.tmp_w * C - 1;
@@ -857,7 +805,7 @@ __global__ void __launch_bounds__(256, C == 1 ? 2 : 1) patch_p12_kernel(LevelGeo
     }
   }
   if (valid) {
-    float* pw = g.pat_w + ((size_t)frame * g.np + ip) * Cfg::N;
+    float* pw = g.pat_w + ((size_t)frame * g.np + ip) * N;
 #pragma unroll
     for (int k = 0; k < NK; ++k) pw[l8 + 8 * k] = wrote_w ? fabsf(R[k]) : 0.f;
     if (l8 == 0) {
@@ -868,6 +816,17 @@ __global__ void __launch_bounds__(256, C == 1 ? 2 : 1) patch_p12_kernel(LevelGeo
       g.pat_cnt[(size_t)frame * g.np + ip] = cnt;
     }
   }
+}
+
+// 8 lanes per patch; dynamic shared memory: the patches' windows, then (RGB) the gradient columns
+template <int NOP, int C>
+void launch_patch_p12(const LevelGeom& g, const PatchParams& pp, int f0, int f1, int init, cudaStream_t st) {
+  using Cfg = PwCfg<NOP, C>;
+  const int threads = 256;
+  const dim3 grid((g.np + threads / 8 - 1) / (threads / 8), f1 - f0);
+  const size_t sm = sizeof(float) * ((size_t)(threads / 8) * Cfg::WIN + (C == 1 ? 0 : (size_t)2 * Cfg::NK * threads));
+  if (sm > 48 * 1024) cudaFuncSetAttribute(patch_p12_kernel<NOP, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+  patch_p12_kernel<NOP, C><<<grid, threads, sm, st>>>(g, pp, f0, init);
 }
 
 // usefbcon, second loop of AggregateFlowDense (patchgrid.cpp:278-375) as a gather: the patches of
@@ -1056,57 +1015,11 @@ int launch_patch_optimize(const LevelGeom& g, const PatchParams& pp, int f0, int
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
   }
   if (g.P == 12 && g.pad >= 12 && (g.noc == 1 || g.noc == 3)) {  // window-staged specialisation (operating points 3 and 4)
-    const int threads12 = 256;
-    const dim3 grid12((g.np + threads12 / 8 - 1) / (threads12 / 8), f1 - f0);
     const int init = init_from_coarser ? 1 : 0;
-    // TMA window fill (option "patch_window_tma"): needs a tensor map over the padded I1 frames, i.e.
-    // row pitch and frame stride multiples of 16 bytes; other levels keep the LDG fill
-    CUtensorMap tmap;
-    memset(&tmap, 0, sizeof(tmap));
-    bool tma = false;
-    // (RGB flow: 32 windows of 17 x 60 floats + the gradient columns exceed an SM's shared memory: LDG fill)
-    const size_t tma_smem = (size_t)(threads12 / 8) * (((g.nop == 2 ? PwCfg<1>::W : PwCfg<1>::P + 1) * PwCfg<1>::WT * g.noc * 4 + 127) / 128 * 128) +
-                            (g.noc == 1 ? 0 : sizeof(float) * 2 * PwCfg<3>::NK * threads12) + 8 * (threads12 / 8);
-    if (pp.window_tma && tma_smem <= 227 * 1024 && ((size_t)g.tmp_w * g.noc * 4) % 16 == 0 && (g.img_fs[3] * 4) % 16 == 0 &&
-        ((uintptr_t)g.img[3]) % 16 == 0) {
-      typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-      static EncodeFn encode = nullptr;
-      if (!encode) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-          encode = (EncodeFn)fn;
-      }
-      if (encode) {
-        const int WH = (g.nop == 2) ? PwCfg<1>::W : PwCfg<1>::P + 1;
-        const int WCB = (g.noc == 1) ? PwCfg<1>::WCB : PwCfg<3>::WCB;
-        const cuuint64_t dims[3] = {(cuuint64_t)g.tmp_w * g.noc, (cuuint64_t)g.tmp_h, (cuuint64_t)f1};
-        const cuuint64_t strides[2] = {(cuuint64_t)g.tmp_w * g.noc * 4, (cuuint64_t)g.img_fs[3] * 4};
-        const cuuint32_t box[3] = {(cuuint32_t)WCB, (cuuint32_t)WH, 1u}, estr[3] = {1u, 1u, 1u};
-        tma = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(g.img[3]), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-      }
-    }
-#define OFDIS_P12(NOPv, Cv, TMAv)                                                                                   \
-  do {                                                                                                             \
-    const size_t sm = sizeof(float) * ((size_t)(threads12 / 8) * PwWin<NOPv, Cv, TMAv>::WIN +                       \
-                                       (Cv == 1 ? 0 : (size_t)2 * PwCfg<Cv>::NK * threads12)) +                    \
-                      (TMAv ? 8 * (threads12 / 8) : 0);                                                            \
-    if (sm > 48 * 1024)                                                                                            \
-      cudaFuncSetAttribute(patch_p12_kernel<NOPv, Cv, TMAv>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); \
-    patch_p12_kernel<NOPv, Cv, TMAv><<<grid12, threads12, sm, st>>>(g, pp, f0, init, tmap);                         \
-  } while (0)
-#define OFDIS_P12T(NOPv, Cv) do { if (tma) OFDIS_P12(NOPv, Cv, true); else OFDIS_P12(NOPv, Cv, false); } while (0)
-    if (g.nop == 2 && g.noc == 1) OFDIS_P12T(2, 1);
-    else if (g.nop == 2) OFDIS_P12T(2, 3);
-    else if (g.noc == 1) OFDIS_P12T(1, 1);
-    else OFDIS_P12T(1, 3);
-#undef OFDIS_P12T
-#undef OFDIS_P12
+    if (g.nop == 2 && g.noc == 1) launch_patch_p12<2, 1>(g, pp, f0, f1, init, st);
+    else if (g.nop == 2) launch_patch_p12<2, 3>(g, pp, f0, f1, init, st);
+    else if (g.noc == 1) launch_patch_p12<1, 1>(g, pp, f0, f1, init, st);
+    else launch_patch_p12<1, 3>(g, pp, f0, f1, init, st);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
   }
   const int n = g.novals;

@@ -394,36 +394,6 @@ def test_lane_sor_and_block_sor_vs_oracle(name, lane, api, oracle_port):
     ctx.close()
 
 
-@pytest.mark.parametrize("name", ["rgb_op3_l1cost_small", "stereo_op4_small"])
-def test_patch_window_filled_by_tma_vs_oracle(name, api, oracle_port):
-    """ofdis_set_option("patch_window_tma", 1): the P = 12 kernel's shared-memory window of I1 comes from a TMA
-    tensor tile copy on the levels whose padded row pitch is a multiple of 16 bytes (here: some levels yes, some
-    no), out-of-image cells zero-filled by the TMA unit -- patch results and the whole run, bitwise."""
-    h, w, ch, mk, amp, stereo = CASES[name]
-    prm = mk()
-    i0, i1, _ = synth.synthetic_pair(h, w, ch, seed=1, amp=amp, stereo=stereo)
-    pyr = preprocess.PairPyramids(i0, i1, prm.sc_f, prm.p_samp_s)
-    ctx = api.Context(prm, pyr.width, pyr.height, pyr.imgpadding, 2)
-    ctx.set_option("patch_window_tma", 1)
-    for f in range(2):
-        ctx.upload_pyramids(f, pyr)
-    lv = prm.sc_l
-    hh, ww = pyr.level_shape(lv + 1)
-    rng = np.random.default_rng(2)
-    fp = (rng.standard_normal((hh, ww, prm.nop)) * 2).astype(np.float32)
-    if stereo:
-        fp = -np.abs(fp)
-    exp = oracle_port.port_level_patches(pyr, prm, lv, fp)
-    ctx.set_flow(1, lv + 1, fp)
-    ctx.patgrid_optimize(lv, 1, 2, True)
-    got = ctx.get_patches(1, lv)
-    for k in ("p", "pweight", "conv", "cnt"):
-        assert_bits(got[k], exp[k], "patch." + k)
-    ctx.run(2)
-    assert_bits(ctx.get_flow(1, prm.sc_l), oracle_port.port_run(pyr, prm), "run")
-    ctx.close()
-
-
 def test_cluster_of_sixteen_bands_where_the_device_grants_it(api, oracle_port):
     """Non-portable cluster size 16: 1100-row level as 9 bands of 64 lanes x 2 rows (all sweeps in flight)."""
     prm = params.from_cli_numbers("1 0 6 6 0.05 0.95 0 8 0.4 0 1 0 1 10 10 5 1 3 1.6 0".split(), noc=1, nop=2)
